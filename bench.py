@@ -18,6 +18,7 @@ Workloads (BASELINE.json configs, SURVEY.md §8d):
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3|c3agg|c2|c1|c4] [--rows R] [--source ...]
     python bench.py --impl reference ...     # the reference algorithm on the host cores (CPU)
+    python bench.py --dump-outputs DIR ...   # also write a seeded sample of the last timed step's merged batch
 
 `value`     whole-job merged (= input) rows/s with the inputs (file bytes / columns) already resident in HBM.
 `e2e`       same metric through the public reader API with HOST buffers: every step copies the Parquet files
@@ -555,6 +556,59 @@ def parity_sample(schema, spec, rd, run_handles, all_keys, n_out, target_rows=30
                        "bit-exact against the oracle's merge of the same input rows"}
 
 
+DUMP_BLOCKS, DUMP_BLOCK_ROWS = 64, 256
+DUMP_MAX_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(schema, merge_handle, n_out, out_dir, seed=0):
+    """--dump-outputs: a fixed, seeded sample of the merged batch the last timed step left on the device, as the host
+    columns SortMergeReader.fetch hands a caller, written as out_dir/<name>.npy so that two builds can be compared
+    output for output.  The sample is DUMP_BLOCKS blocks of DUMP_BLOCK_ROWS consecutive rows at seeded positions
+    (every row when the batch is smaller).  For each file column <name>:
+      <name>.npy                      fixed-width values as float64, 0 under NULL; an INT64 column, which float64
+                                      cannot hold exactly, becomes <name>.hi32.npy (signed upper 32 bits) and
+                                      <name>.lo32.npy (unsigned lower 32 bits)
+      <name>.len.npy, <name>.bytes.npy  var-len columns: byte length of every value (0 under NULL, float64) and the
+                                      values' bytes back to back (float32)
+      <name>.valid.npy                nullable columns: 1.0 where the value is present (float32)
+    and row_index.npy (the sampled row positions) and rows_out.npy (the batch's row count)."""
+    from paimon_b200.columnar import unpack_validity
+    from paimon_b200.sort_merge_reader import fetch_slice
+    from paimon_b200.types import PhysicalType, is_varlen, numpy_dtype
+    if n_out <= DUMP_BLOCKS * DUMP_BLOCK_ROWS:
+        starts, block = ([0] if n_out else []), n_out
+    else:
+        slots = np.random.default_rng(seed).choice(n_out // DUMP_BLOCK_ROWS, DUMP_BLOCKS, replace=False)
+        starts, block = sorted(int(s) * DUMP_BLOCK_ROWS for s in slots), DUMP_BLOCK_ROWS
+    parts = [fetch_slice(schema, merge_handle, s, s + block) for s in starts]
+
+    def cat(arrays, dtype):
+        return np.concatenate(arrays).astype(dtype) if arrays else np.zeros(0, dtype)
+    out = {"row_index": cat([np.arange(s, s + block) for s in starts], np.float64),
+           "rows_out": np.array([n_out], np.float64)}
+    for ci, f in enumerate(schema.file_fields()):
+        cols = [p.columns[ci].canonical() for p in parts]
+        if f.nullable:
+            out[f"{f.name}.valid"] = cat([unpack_validity(c.valid, len(c)) for c in cols], np.float32)
+        if is_varlen(f.physical):
+            out[f"{f.name}.len"] = cat([np.diff(c.offsets.astype(np.int64)) for c in cols], np.float64)
+            out[f"{f.name}.bytes"] = cat([c.data for c in cols], np.float32)
+        elif f.physical == PhysicalType.INT64:
+            v = cat([c.data for c in cols], np.int64)
+            out[f"{f.name}.hi32"] = (v >> 32).astype(np.float64)
+            out[f"{f.name}.lo32"] = (v & 0xFFFFFFFF).astype(np.float64)
+        else:
+            out[f.name] = cat([c.data for c in cols], numpy_dtype(f.physical)).astype(np.float64)
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit(f"--dump-outputs: the sample takes {total} bytes, more than {DUMP_MAX_BYTES}")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    print(f"--dump-outputs: {len(out)} arrays, {total} bytes, {len(out['row_index'])} of {n_out} merged rows -> {out_dir}",
+          file=sys.stderr)
+
+
 # ------------------------------------------------------------------ main
 
 def main():
@@ -579,7 +633,11 @@ def main():
     ap.add_argument("--no-parity-sample", action="store_true")
     ap.add_argument("--cpu-sample-rows", type=int, default=None)
     ap.add_argument("--cpu-threads", type=int, default=None)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write a seeded sample of the last step's merged batch to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -747,6 +805,9 @@ def main():
         wall = time.perf_counter() - t0
         clocks = sampler.stop()
         dev_ms = e0.elapsed_time(e1)
+
+    if args.dump_outputs and rank == 0:
+        dump_outputs(schema, rd._merge_h, int(s.rows_out), args.dump_outputs)
 
     t = torch.tensor([dev_ms], device=dev, dtype=torch.float64)
     if world > 1:
